@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm, config C1 (the one the metric is quoted on)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port), same config
     python bench.py --config C2|C3|C4|C5 [--rows R]          # the other BASELINE.json configs, at size
+    python bench.py --steps K --warmup W --dump-outputs DIR  # C1, plus what the last timed steps returned, as .npy
 
 C1 (default; what the driver runs): a "step" is ONE complete IVF_PQ(256,16) index build over the
 1M x 128 f32 dataset: sample -> k-means (IVF) -> residuals -> 16 sub-space k-means (PQ) -> partition id +
@@ -307,6 +308,28 @@ KERNEL_BYTES = {
 }
 
 
+DUMP_ROWS = 1 << 19   # storage positions of codes / row ids kept by --dump-outputs (about 40 MB in all at C1)
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: DIR/<name>.npy; float32 and integers of <= 16 bits as float32, the rest as float64 (exact:
+    row ids and offsets are below 2**53)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        small = a.dtype == np.float32 or (a.dtype.kind in "iu" and a.dtype.itemsize <= 2)
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32 if small else np.float64))
+
+
+def build_outputs(parts):
+    """What a caller of the build receives (lb2_index_export); codes and row ids at a fixed, seeded sample of
+    storage positions when there are more than DUMP_ROWS rows."""
+    n = len(parts["row_ids"])
+    pos = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False)) if n > DUMP_ROWS else slice(None)
+    return {"centroids": parts["centroids"], "codebook": parts["codebook"], "part_offsets": parts["part_offsets"],
+            "codes": parts["codes"][pos], "row_ids": parts["row_ids"][pos]}
+
+
 def load_ncu_traffic():
     """dram__bytes_read.sum + dram__bytes_write.sum per launch from the committed `ncu --set full` summary
     of the same kernels on the same workload (profiles/ncu_traffic.json, written by profiles/summarize_ncu.py)"""
@@ -327,7 +350,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only", default="all", choices=["all", "build", "query"],
                     help="profiling aid (ncu): restrict the run to the resident build or to the query batch")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed build step and the last timed search batch returned as "
+                         "DIR/<name>.npy (rank 0; the inputs are the same on every run with the same arguments)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.config != "C1" or args.impl != "ours"):
+        ap.error("--dump-outputs is defined on our arm of config C1")
     if args.config != "C1":
         if args.steps is None:
             args.steps = 2
@@ -399,15 +427,22 @@ def main():
     lb.launch_count(reset=True)
     t_wall0 = time.time()
     lb.timer_start()
-    stats = None
-    for _ in range(args.steps):
+    stats = last = None
+    for i in range(args.steps):
         ix = lb.IvfPqIndex.build(data_dev, "l2", params, row_ids=rid_dev)
         stats = ix.stats
-        ix.close()
+        if args.dump_outputs and i == args.steps - 1:
+            last = ix   # exported after the timed window
+        else:
+            ix.close()
     ms_total = lb.timer_stop()
     barrier()
     t_wall1 = time.time()
     launches = lb.launch_count()
+    dumped = {}
+    if last is not None:
+        dumped = build_outputs(last.export())
+        last.close()
     ms_step = max_over_ranks(ms_total / args.steps)
     clocks = sampler.summary(t_wall0, t_wall1)
     value = world * n / (ms_step * 1e-3) / 1e6
@@ -462,6 +497,8 @@ def main():
     if args.only == "build":
         if rank == 0:
             print(json.dumps({"only": "build", "ms_per_step": ms_step, "value": value, "kernels": fams}))
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, dumped)
         return
     # ---- e2e build: pinned host -> device -> host, through the C ABI ---------------------------
     e2e = None
@@ -521,6 +558,8 @@ def main():
     q_ms = max_over_ranks(lb.timer_stop() / args.steps)
     barrier()
     lb.profile.enable(False)
+    if args.dump_outputs:
+        dumped.update(search_ids=ids_t.cpu().numpy(), search_dists=d_t.cpu().numpy())
     scan_name = "search:pq_scan_skew"                      # the conflict-free persistent scan (large batches)
     scan_cnt, scan_ms = lb.profile.get(scan_name)
     if scan_cnt == 0:
@@ -645,6 +684,8 @@ def main():
             "query_table": query_table, "query_replica": query_replica, "cpu_baseline": cpu_baseline,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         from lance_b200 import parallel
         parallel.comm_destroy()

@@ -1,7 +1,7 @@
 """The oracle (oracle/lance_oracle.cc) against the reference's own known-answer tests
 (tests/golden/reference_known_answers.json, transcribed by tests/golden/make_known_answers.py)
-and against the two reference C kernels compiled from /root/reference (oracle/_ref)."""
-import ctypes as C
+and against the outputs of two reference C kernels on fixed inputs (tests/golden/ref_simd_outputs.npz,
+recorded by tests/golden/make_ref_simd_outputs.py)."""
 import json
 import os
 
@@ -12,6 +12,7 @@ from oracle import binding as ob
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CASES = json.load(open(os.path.join(HERE, "golden", "reference_known_answers.json")))
+REF_SIMD = np.load(os.path.join(HERE, "golden", "ref_simd_outputs.npz"))
 
 
 def _check(got, c):
@@ -87,17 +88,11 @@ def test_l2_lane_order_is_reference_order():
 
 
 def test_f16_l2_against_reference_c_kernel():
-    so = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "libref_simd.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref not built (reference sources absent)")
-    ref = C.CDLL(so)
-    ref.l2_f16_avx2.restype = C.c_float
-    ref.l2_f16_avx2.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
-    rng = np.random.default_rng(1)
-    for d in (8, 16, 128, 130, 768):
-        x = rng.standard_normal(d).astype(np.float16)
-        y = rng.standard_normal(d).astype(np.float16)
-        r = ref.l2_f16_avx2(x.ctypes.data, y.ctypes.data, d)
+    """the reference's l2_f16_avx2 (f16.c) on fixed inputs: its outputs are stored in REF_SIMD"""
+    assert list(REF_SIMD["f16_dims"]) == [8, 16, 128, 130, 768]
+    for d in REF_SIMD["f16_dims"]:
+        x, y = REF_SIMD[f"f16_x_{d}"], REF_SIMD[f"f16_y_{d}"]
+        r = float(REF_SIMD[f"f16_l2_{d}"])
         o = ob.l2_f16(x, y)
         # the C kernel is built -ffast-math (build.rs:99): association unspecified -> tolerance
         assert abs(r - o) <= 1e-5 * max(abs(r), 1e-6)
@@ -122,27 +117,16 @@ def test_sum_4bit_dist_table_known_answer(c):
 
 
 def test_sum_4bit_dist_table_against_reference_c_kernel():
-    """oracle/_ref's dist_table.o is the reference's own AVX-512 kernel (dist_table.c:8): bit-equal to
+    """the reference's own AVX-512 kernel (dist_table.c:8), whose outputs are stored in REF_SIMD: bit-equal to
     the restatement on the reference literal and on random codes (integer arithmetic)."""
-    so = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "libref_simd.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref not built (reference sources absent)")
-    flags = open("/proc/cpuinfo").read()
-    if "avx512bw" not in flags:
-        pytest.skip("host CPU has no AVX-512BW")
-    ref = C.CDLL(so)
-    ref.sum_4bit_dist_table_32bytes_batch_avx512.restype = None
-    ref.sum_4bit_dist_table_32bytes_batch_avx512.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
-    rng = np.random.default_rng(7)
-    cases = [(np.asarray(c["codes"], np.uint8), np.asarray(c["dist_table"], np.uint8), c["code_len"])
-             for c in CASES if c["op"] == "sum_4bit_dist_table"]
-    for code_len in (2, 4, 8, 16):  # the C kernel consumes 64 code bytes (= 2 sub-vector pairs) per step
-        cases.append((rng.integers(0, 256, 32 * code_len, dtype=np.uint8),
-                      rng.integers(0, 256 // (2 * code_len), 32 * code_len, dtype=np.uint8), code_len))
-    for codes, table, code_len in cases:
-        out = np.zeros(32, np.uint16)
-        ref.sum_4bit_dist_table_32bytes_batch_avx512(codes.ctypes.data, codes.size, table.ctypes.data, out.ctypes.data)
-        assert np.array_equal(out, ob.sum_4bit_dist_table(32, code_len, codes, table)), code_len
+    lit = [c for c in CASES if c["op"] == "sum_4bit_dist_table"]
+    n = int(REF_SIMD["dt_cases"])
+    assert n == len(lit) + 4
+    for i in range(n):
+        codes, table, code_len = REF_SIMD[f"dt_codes_{i}"], REF_SIMD[f"dt_table_{i}"], int(REF_SIMD[f"dt_code_len_{i}"])
+        if i < len(lit):
+            assert np.array_equal(codes, lit[i]["codes"]) and np.array_equal(table, lit[i]["dist_table"])
+        assert np.array_equal(REF_SIMD[f"dt_sum_{i}"], ob.sum_4bit_dist_table(32, code_len, codes, table)), code_len
 
 
 def test_range_query_follows_flat_index_semantics():
